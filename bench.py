@@ -473,8 +473,14 @@ def workload_name(workload, quant):
             f"greedy completion")
 
 
-def measure(dsk, torch, dist, w, rank, world, local_rank, steps, warmup, want_e2e=True, profile=False):
-    """Mints the workload on this rank's GPU and times `steps` completions: returns a dict (rank-local; times are max over ranks)."""
+# --dump-outputs: the e2e path returns GEN_TOKENS x vocab logits per completion; a fixed sample of vocabulary columns keeps the
+# dump small (V3: 128 x 129280 fp32 would be 66 MB)
+DUMP_VOCAB_SAMPLE = 8192
+
+
+def measure(dsk, torch, dist, w, rank, world, local_rank, steps, warmup, want_e2e=True, profile=False, keep_outputs=False):
+    """Mints the workload on this rank's GPU and times `steps` completions: returns a dict (rank-local; times are max over ranks).
+    keep_outputs: also return what the last timed completion of each path handed back (res["outputs"], name -> array)."""
     m = mint_on_gpu(dsk, w, rank, world, local_rank)
     log(f"rank {rank}/{world}: minted {m.resident_bytes() / 1e9:.2f} GB resident, {m.active_bytes_per_token() / 1e9:.3f} GB/token algorithmic")
     if world > 1:
@@ -546,20 +552,31 @@ def measure(dsk, torch, dist, w, rank, world, local_rank, steps, warmup, want_e2
 
     # ---- e2e: reference-shaped host loop, host buffers, copies inside the timed region -------------
     e2e = None
+    outputs = {"tokens": toks.astype(np.float64)} if keep_outputs else None
     if want_e2e:
-        def host_completion():
+        cols = np.sort(np.random.default_rng(0).choice(vocab, min(vocab, DUMP_VOCAB_SAMPLE), replace=False))
+
+        def host_completion(keep=False):
             am = hydrate()
             t0 = time.perf_counter()
             pos = PROMPT_LEN
+            kept_tokens, kept_logits = [], []
             for _ in range(GEN_TOKENS):
                 logits, _ = m.forward(am, pos)            # H2D control words, D2H vocab logits, sync
                 am = int(np.argmax(logits))               # host sampler (Sampler::sample_argmax)
+                if keep:
+                    kept_tokens.append(am)
+                    kept_logits.append(logits[cols])
                 pos += 1
-            return time.perf_counter() - t0
+            elapsed = time.perf_counter() - t0
+            if keep:
+                outputs.update(e2e_tokens=np.array(kept_tokens, np.float64), e2e_logits=np.stack(kept_logits),
+                               e2e_logits_vocab_index=cols.astype(np.float64))
+            return elapsed
         for _ in range(max(1, warmup // 2)):
             host_completion()
         barrier()
-        e2e_s = sum(host_completion() for _ in range(steps))
+        e2e_s = sum(host_completion(keep=keep_outputs and i + 1 == steps) for i in range(steps))
         if dist is not None:
             t = torch.tensor([e2e_s], device="cuda")
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -568,7 +585,7 @@ def measure(dsk, torch, dist, w, rank, world, local_rank, steps, warmup, want_e2
         log(f"e2e {e2e:.1f} tok/s")
     res = {"value": value, "dev_ms": dev_ms, "wall": wall, "e2e": e2e, "clocks": clk, "sharded_check": sharded_check,
            "abytes": m.active_bytes_per_token(), "resident_gb": m.resident_bytes() / 1e9, "tokens": toks[:8].tolist(),
-           "launches_per_forward": m.launches_per_forward(dsk.OUTPUT_LOGITS), "timeline": timeline}
+           "launches_per_forward": m.launches_per_forward(dsk.OUTPUT_LOGITS), "timeline": timeline, "outputs": outputs}
     m.close()
     torch.cuda.empty_cache()
     return res
@@ -612,7 +629,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the V2-Lite configs[1]/[2] continuity numbers")
     ap.add_argument("--profile-token", action="store_true", help="print the per-stage timeline of one token to stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed completion returned as DIR/<name>.npy: tokens (device loop), e2e_tokens and "
+                         "e2e_logits (host loop, at the vocabulary columns in e2e_logits_vocab_index); inputs are seeded")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -657,7 +679,13 @@ def main():
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     dsk.init(local_rank)
     log(f"rank {rank}/{world}: workload {a.workload}/{a.quant}")
-    R = measure(dsk, torch, dist, w, rank, world, local_rank, a.steps, a.warmup, want_e2e=True, profile=a.profile_token)
+    R = measure(dsk, torch, dist, w, rank, world, local_rank, a.steps, a.warmup, want_e2e=True, profile=a.profile_token,
+                keep_outputs=bool(a.dump_outputs) and rank == 0)
+    if R["outputs"]:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        for name, arr in R["outputs"].items():
+            np.save(os.path.join(a.dump_outputs, name + ".npy"), arr)
+        log(f"outputs of the last timed step written to {a.dump_outputs}: {sorted(R['outputs'])}")
 
     if rank != 0:
         if dist is not None:

@@ -1,6 +1,6 @@
 """GPU parity of the true-MLA blocks (checkpoints converted with --mla: BlockMLA::_attention_impl src/infer.cpp:1051-1141,
-attn_mla 766-804) against the UNMODIFIED reference (oracle/_ref): latent + rope KV caches bit-compared after teacher-forced
-tokens, tier T2 (every layer re-synchronised on the checker's input and caches) and tier T3 (teacher-forced logits), the
+attn_mla 766-804) against the UNMODIFIED reference (oracle/_ref) or, where that is absent, the C restatement: latent + rope
+KV caches bit-compared after teacher-forced tokens, tier T2 (every layer re-synchronised on the checker's input and caches) and tier T3 (teacher-forced logits), the
 in-kernel token loop, and the sink re-rotation past rope_scaling_original_max_position_embeddings."""
 import os
 import shutil
@@ -30,11 +30,6 @@ def dsk():
     return d
 
 
-def _need_ref():
-    if O.ref_lib() is None:
-        pytest.skip("oracle/_ref is not built (make -C oracle ref): the port has no BlockMLA restatement")
-
-
 def _mint(preset, quant, **kw):
     d = tempfile.mkdtemp(prefix=f"dsk_mla_{preset}_{quant}_")
     if quant == "f8e5m2":
@@ -49,7 +44,6 @@ CASES = [("tiny_v2", "fp32"), ("tiny_v3", "fp32"), ("tiny_v2", "fp16"), ("tiny_v
 
 @pytest.mark.parametrize("preset,quant", CASES)
 def test_mla_layers_caches_and_logits(dsk, preset, quant):
-    _need_ref()
     d = _mint(preset, quant)
     try:
         m = dsk.Model.from_dir(d)
@@ -140,7 +134,6 @@ def test_mla_e2e_golden(dsk, golden_dir, tmp_path):
 def test_mla_sinks_past_original_max(dsk):
     """pos >= rope_scaling_original_max_position_embeddings: 2 sink rows, ring positions, sink rope keys re-rotated by one
     position per step (src/infer.cpp:1099-1111) — teacher-forced against the reference through 8 steps past the limit."""
-    _need_ref()
     d = tempfile.mkdtemp(prefix="dsk_mla_sink_")
     try:
         mint.mint(d, "tiny_v3", "fp32", use_mla=True, fast=True, original_max_position=12, max_seq_len=16)
@@ -167,7 +160,6 @@ def test_mla_sinks_past_original_max(dsk):
 def test_mla_long_context(dsk):
     """700 cached positions (several passes of every loop of the attention stage: scores 8 positions per round, softmax and
     latent mix 256 per round), teacher-forced against the reference; logits compared every 100 tokens and on the last 10."""
-    _need_ref()
     d = tempfile.mkdtemp(prefix="dsk_mla_long_")
     try:
         mint.mint(d, "tiny_v2", "fp16", use_mla=True, fast=True, max_seq_len=1024)

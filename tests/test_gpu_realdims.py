@@ -8,7 +8,7 @@
 (and, for two cases, the same dims converted with --mla: true-MLA blocks) each as 1 dense + 1 MoE layer + LM head (first_k_dense_replace overridden to 1 so both layer kinds appear).  The tiny
 presets exercise every branch of the algorithm; this file exercises the production TILE SHAPES of the interpreter at these
 dims (K-quant rows of 1536 / 5120 / 7168 / 16384 / 18432 columns, 128-head attention, E = 160 / 256 routing, 0.5-0.9 M-row
-LM heads) against the unmodified reference (oracle/_ref), tiers T2 (re-synchronised layers) and T3 (teacher-forced)."""
+LM heads) against the unmodified reference (oracle/_ref) or, where that is absent, the C restatement, tiers T2 (re-synchronised layers) and T3 (teacher-forced)."""
 import os
 import shutil
 import tempfile
@@ -54,8 +54,6 @@ def _mint(workload, quant, n_layers=2, mla=False):
 def test_real_dims_layers_and_logits(dsk, workload, quant, mla):
     """mla=True: the same dims converted with --mla (BlockMLA): 128 heads x (512-wide latent + 64 rope) attention, the
     65536 x 1536 absorbed projection wc, per-head 128 x 512 wv_b slabs."""
-    if mla and O.ref_lib() is None:
-        pytest.skip("BlockMLA parity needs oracle/_ref")
     d = _mint(workload, quant, mla=mla)
     try:
         m = dsk.Model.from_dir(d)

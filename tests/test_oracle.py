@@ -1,5 +1,5 @@
-"""CPU suite: pins the oracle restatement against the committed golden vectors and (when oracle/_ref is built)
-against the unmodified reference itself; checks host logic and that libdsk.so exports the declared C-ABI."""
+"""CPU suite: pins the oracle restatement against golden vectors committed from the unmodified reference; checks host logic
+and that libdsk.so exports the declared C-ABI."""
 import ctypes
 import json
 import os
@@ -12,8 +12,6 @@ import oracle as O
 from conftest import rel_l2
 
 P = O.Ops("port")
-HAVE_REF = O.ref_lib() is not None
-needs_ref = pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref/libdsref.so not built")
 
 
 @pytest.fixture(scope="module")
@@ -147,108 +145,87 @@ def test_e2e_mla_golden_port(golden_dir, tmp_path):
                     assert np.allclose(a, b, rtol=2e-3, atol=1e-4), (key, name)
 
 
-# ---- port vs the unmodified reference, live (build container and GPU box both carry oracle/_ref) ----
-@needs_ref
-def test_q8k_bit_exact_vs_ref():
-    R = O.Ops("ref")
-    rng = np.random.default_rng(5)
-    for t in range(100):
-        x = (rng.standard_normal(1024) * 10 ** rng.uniform(-4, 4)).astype(np.float32)
-        a, b = R.quantize_q8k(x).reshape(-1, 292), P.quantize_q8k(x).reshape(-1, 292)
-        assert np.array_equal(a, b)
+# ---- port vs the unmodified reference (its outputs committed: tests/golden/make_golden_port.py) ----------
+@pytest.fixture(scope="module")
+def pvr(golden_dir):
+    return np.load(os.path.join(golden_dir, "port_vs_ref.npz"))
 
 
-@needs_ref
+def _logits(s, pvr):
+    return s.buffer("logits")[pvr["logit_idx"]]
+
+
+def test_q8k_bit_exact_vs_ref(pvr):
+    from golden.make_golden_port import digest, q8k_inputs
+    for t, x in enumerate(q8k_inputs()):
+        assert np.array_equal(digest(P.quantize_q8k(x)), pvr["q8k_sha256"][t]), t
+
+
 @pytest.mark.parametrize("quant,tol", [("fp32", 1e-5), ("fp16", 1e-6), ("f8e5m2", 1e-6), ("q2_k", 2e-6), ("q3_k", 2e-6)])
-def test_gemv_vs_ref(quant, tol):
-    import mint
-    R = O.Ops("ref")
-    rng = np.random.default_rng(6)
-    d, n = 96, 1024
-    w = (rng.standard_normal((d, n)) * n ** -0.5).astype(np.float32)
-    x = rng.standard_normal(n).astype(np.float32)
-    scale = None
-    if quant == "fp16":
-        wq = w.astype(np.float16)
-    elif quant == "f8e5m2":
-        wq, scale = mint.f8e5m2_blockwise(w)
-    elif quant in ("q2_k", "q3_k"):
-        wq = mint.kquant_rows(w, quant, False, rng)
-    else:
-        wq = w
-    assert rel_l2(P.matmul(x, wq, quant, d, n, scale), R.matmul(x, wq, quant, d, n, scale)) < tol
+def test_gemv_vs_ref(pvr, quant, tol):
+    from golden.make_golden_port import gemv_inputs
+    assert rel_l2(P.matmul(*gemv_inputs(quant)), pvr[f"gemv_{quant}"]) < tol
 
 
-@needs_ref
 @pytest.mark.parametrize("preset", ["tiny_v2lite", "tiny_v2", "tiny_v3"])
 @pytest.mark.parametrize("quant,tol", [("fp32", 1e-3), ("f8e5m2", 1e-3), ("q3_k", 5e-2)])
-def test_forward_port_vs_ref(ckpt, preset, quant, tol):
-    d = ckpt(preset, quant)
-    r, p = O.RefSession(d), O.PortSession(d)
-    for pos, tok in enumerate([0, 9, 400, 33, 1001]):
-        r.forward(tok, pos)
+def test_forward_port_vs_ref(ckpt, pvr, preset, quant, tol):
+    from golden.make_golden_port import FORWARD_MINT_KW, FORWARD_TOKENS
+    p = O.PortSession(ckpt(preset, quant, **FORWARD_MINT_KW))
+    exp = pvr[f"forward_{preset}_{quant}_logits"]
+    for pos, tok in enumerate(FORWARD_TOKENS):
         p.forward(tok, pos)
-        assert rel_l2(p.buffer("logits"), r.buffer("logits")) < tol
-    r.close()
+        assert rel_l2(_logits(p, pvr), exp[pos]) < tol
 
 
-@needs_ref
 @pytest.mark.parametrize("preset", ["tiny_v2", "tiny_v3"])
 @pytest.mark.parametrize("quant,tol", [("fp32", 1e-3), ("fp16", 1e-3), ("f8e5m2", 1e-3), ("q2_k", 1.5e-1)])   # (q2_k T3: sanity
 # ceiling only — one Q8_K rounding flip between the two builds moves random-block logits by several 1e-2, see
 # profiles/r02_reference_self_sensitivity.txt; the T2 part below is the proof)
-def test_mla_block_port_vs_ref(ckpt, preset, quant, tol):
-    """BlockMLA, layer by layer on the reference's input and caches (tier T2), then teacher-forced logits (T3)."""
-    kw = {"v_head_dim": 128} if quant == "f8e5m2" else {}
-    d = ckpt(preset, quant, use_mla=True, **kw)
-    r, p = O.RefSession(d), O.PortSession(d)
-    errs = []
-    for pos, tok in enumerate([0, 9, 400, 33]):
-        r.copy_embedding(tok)
+def test_mla_block_port_vs_ref(ckpt, pvr, preset, quant, tol):
+    """BlockMLA, layer by layer on the reference's cache rows, each layer against the reference's output for the same input
+    (tier T2), then teacher-forced logits (T3)."""
+    from golden.make_golden_port import FORWARD_TOKENS, MLA_T2_TOKENS, mla_mint_kw
+    d = ckpt(preset, quant, **mla_mint_kw(quant))
+    key = f"mla_{preset}_{quant}"
+    p = O.PortSession(d)
+    xi, n_layers, errs = pvr["x_idx"], p.c["n_layers"], []
+    for pos, tok in enumerate(MLA_T2_TOKENS):
         p.copy_embedding(tok)
-        for l in range(p.c["n_layers"]):
-            p.buffer("x")[:] = r.buffer("x")
-            for which in (0, 1):
-                p.kv_cache(l, which)[:] = r.kv_cache(l, which)
-            r.block(l, pos, 0, pos, pos + 1)
+        for l in range(n_layers):
+            for which, name in ((0, "_t2_latent"), (1, "_t2_rope")):
+                rows = pvr[key + name][l]
+                p.kv_cache(l, which)[:rows.size] = rows
             p.block(l, pos, 0, pos, pos + 1)
-            errs.append(rel_l2(p.buffer("x"), r.buffer("x")))
+            errs.append(rel_l2(p.buffer("x")[xi], pvr[key + "_t2_x"][pos * n_layers + l]))
     errs = np.array(errs)
     if quant == "q2_k":   # Q8_K rounding flips between the two builds (-O3 -ffast-math vs -O2): most pairs clean, flips bounded
         assert np.median(errs) < 1e-5 and errs.max() < 5e-2, errs
     else:
         assert errs.max() < 1e-4, errs
-    r.close()
-    r, p = O.RefSession(d), O.PortSession(d)
-    for pos, tok in enumerate([0, 9, 400, 33, 1001]):
-        r.forward(tok, pos)
+    p = O.PortSession(d)
+    for pos, tok in enumerate(FORWARD_TOKENS):
         p.forward(tok, pos)
-        assert rel_l2(p.buffer("logits"), r.buffer("logits")) < tol, (preset, quant, pos)
-    r.close()
+        assert rel_l2(_logits(p, pvr), pvr[key + "_logits"][pos]) < tol, (preset, quant, pos)
 
 
-@needs_ref
-def test_mla_sink_ring_port_vs_ref(ckpt):
+def _sink_ring(ckpt, pvr, name):
+    from golden.make_golden_port import SINK_STEPS, sink_mint_kw
+    preset, kw = sink_mint_kw(name)
+    p = O.PortSession(ckpt(preset, "fp32", **kw))
+    for pos in range(SINK_STEPS):
+        p.forward(pos * 7 % 1024, pos)
+        assert rel_l2(_logits(p, pvr), pvr[f"{name}_logits"][pos]) < 1e-3, pos
+
+
+def test_mla_sink_ring_port_vs_ref(ckpt, pvr):
     """MLA past original_max_position: 2 sink rows, ring overwrite, sink rope keys re-rotated (src/infer.cpp:1099-1111)."""
-    d = ckpt("tiny_v3", "fp32", use_mla=True, original_max_position=8)
-    r, p = O.RefSession(d), O.PortSession(d)
-    for pos in range(14):
-        r.forward(pos * 7 % 1024, pos)
-        p.forward(pos * 7 % 1024, pos)
-        assert rel_l2(p.buffer("logits"), r.buffer("logits")) < 1e-3, pos
-    r.close()
+    _sink_ring(ckpt, pvr, "mla_sink")
 
 
-@needs_ref
-def test_sink_ring_port_vs_ref(ckpt):
+def test_sink_ring_port_vs_ref(ckpt, pvr):
     """pos >= original_max_position: 2 sinks kept, ring overwrite, sink keys re-rotated (src/infer.cpp:1271-1277, 1008-1020)."""
-    d = ckpt("tiny_v2lite", "fp32", original_max_position=8)
-    r, p = O.RefSession(d), O.PortSession(d)
-    for pos in range(14):
-        r.forward(pos * 7 % 1024, pos)
-        p.forward(pos * 7 % 1024, pos)
-        assert rel_l2(p.buffer("logits"), r.buffer("logits")) < 1e-3, pos
-    r.close()
+    _sink_ring(ckpt, pvr, "sink")
 
 
 # ---- host logic -------------------------------------------------------------------------------------
